@@ -2,6 +2,8 @@
 
     python bench.py --gpus N --steps K --warmup W            # this engine (one process per GPU; torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy (same
+                                                             # arguments -> same inputs: compare two builds output for output)
 
 One "step" = sample(B) -> train_policy_on_batch -> soft_target_updates (base_runner.py:259-284) on synthetic
 SMAC-shaped replay data.  Prints ONE JSON line (rank 0).
@@ -59,6 +61,45 @@ def peaks():
         d = json.load(open(path))
         return dict(hbm=d["hbm_gbs"], tflops=d["bf16_tflops"], tflops_sustained=d.get("bf16_tflops_sustained", d["bf16_tflops"]), src="measured")
     return dict(hbm=6650.0, tflops=1590.0, tflops_sustained=1400.0, src="fallback")
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(outdir, arrays):
+    """--dump-outputs: what the timed path computed in its last step, one <outdir>/<name>.npy per array (float64 where the engine keeps
+    float64 or integers, float32 otherwise), so that two builds run with the same arguments can be compared output for output.  An array
+    larger than its share of DUMP_BYTES is cut to a fixed, seeded sample of its elements (the same positions in every run)."""
+    os.makedirs(outdir, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(arrays))
+    for name, a in arrays.items():
+        a = np.asarray(a.detach().cpu() if torch.is_tensor(a) else a)
+        a = a.astype(np.float64 if a.dtype in (np.float64, np.int64) else np.float32)
+        if a.nbytes > share:
+            pos = np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))
+            a = a.reshape(-1)[pos]
+        np.save(os.path.join(outdir, name + ".npy"), a)
+
+
+def qmix_outputs(tr, rep, B):
+    """What the caller of one QMIX / M_QMix step holds afterwards: its train_info, the replay indices it sampled, the new PER priorities
+    and importance weights, and the live and target parameters (the policy's networks are views of them)."""
+    out = dict(loss=tr._info[0], grad_norm=tr._info[1], Q_tot=tr._info[2], sample_indices=rep.sampled_indices(B), params=tr.theta,
+               target_params=tr.theta_tgt)
+    if tr.use_per:
+        out.update(priorities=tr._prio_view[:B], importance_weights=rep.sampled_weights(B))
+    return out
+
+
+def maddpg_outputs(tr, rep, B):
+    """The same for one R-MADDPG / R-MATD3 update; the actor's loss and gradient norm only when that update trained the actor."""
+    pol, info = tr.policies["policy_0"], tr._info
+    out = dict(critic_loss=info[0], critic_grad_norm=info[1], sample_indices=rep.sampled_indices(B),
+               actor_params=pol.actor_vecs[0], target_actor_params=pol.actor_vecs[1], critic_params=pol.critic_vecs[0],
+               target_critic_params=pol.critic_vecs[1])
+    if (tr.num_updates["policy_0"] - 1) % tr.actor_update_interval == 0:
+        out.update(actor_loss=info[4], actor_grad_norm=info[5])
+    return out
 
 
 MADDPG_WORKLOADS = {
@@ -171,6 +212,8 @@ def run_maddpg(args):
     ms = e0.elapsed_time(e1) / args.steps
     launches = int(lib.mx_launch_count() - l0)
     torch.cuda.synchronize()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, maddpg_outputs(tr, buf.policy_buffers["policy_0"], B))
     if args.quick:          # tuning sweeps: the device-resident number only (not a bench line)
         emit(dict(quick=True, workload=args.workload, value=1000.0 / ms, ms_per_step=ms, opts=args.opt, kernels_per_step=launches / args.steps))
         return
@@ -509,6 +552,8 @@ def run_engine(args):
     if world > 1:
         torch.distributed.all_reduce(ms_total, op=torch.distributed.ReduceOp.MAX)
     ms_step = float(ms_total) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, qmix_outputs(tr, pb, B))
     exchange = None
     if p2p:
         # per rank: mean us per step spent pushing the gradient to the peers (+ system fence), waiting for the last peer's flag (rank skew +
@@ -836,6 +881,8 @@ def run_mlp(args):
         torch.cuda.synchronize()
     ms_step = e0.elapsed_time(e1) / args.steps
     launches = int(lib.mx_launch_count() - launches0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, qmix_outputs(tr, rep, B))
     if args.quick:
         emit(dict(quick=True, workload=args.workload, value=1000.0 / ms_step, ms_per_step=ms_step, opts=args.opt, kernels_per_step=graph.num_kernels))
         graph.close()
@@ -947,7 +994,12 @@ def main():
     ap.add_argument("--buffer", type=int, default=5000, help="replay episodes (scripts/train_smac_qmix.sh default 5000)")
     ap.add_argument("--quick", action="store_true", help="device-resident timing only (tuning sweeps; not the bench contract line)")
     ap.add_argument("--opt", action="append", default=[], help="engine option name=int (mx_set_option), e.g. --opt pdl=0 --opt front_tc=0")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the engine's outputs; the reference arm has none")
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.impl != "reference" and a.opt:
         from offpolicy._b200 import capi
         for kv in a.opt:

@@ -31,6 +31,7 @@ class StepGraph(object):
         g = C.c_void_p()
         capi.check(lib.mx_graph_capture(pb.handle, trainer.handle, int(batch_size), float(beta), self.flags, self._sp, C.byref(g)))
         self.handle = g
+        self.lib = lib          # the library that made the graph frees it, whichever build is bound later
         self.num_kernels = int(lib.mx_graph_num_kernels(g))
         self._keep = (buffer, trainer)
         self._per, self._rep, self._beta = per, pb, float(beta)
@@ -49,7 +50,7 @@ class StepGraph(object):
 
     def close(self):
         if self.handle:
-            capi.lib().mx_graph_destroy(self.handle)
+            self.lib.mx_graph_destroy(self.handle)
             self.handle = None
 
     def __del__(self):

@@ -133,6 +133,7 @@ class QMix(object):
         capi.check(lib.mx_qmix_create(C.byref(self.cfg), capi.ptr(self.theta), capi.ptr(self.theta_tgt), capi.ptr(self.adam_m),
                                       capi.ptr(self.adam_v), capi.ptr(self.workspace), nbytes, C.byref(h)))
         self.handle = h
+        self._lib = lib         # the library that made the handle (and the step graphs) frees them, whichever build is bound later
         self._host_batch = None
         self.use_step_graph = True          # replay the captured launch sequence for batches that live in a replay's batch region
         self._graphs, self._graph_keep, self._cap_stream = {}, [], None
@@ -220,7 +221,7 @@ class QMix(object):
         try:
             self.drop_step_graphs()
             if getattr(self, "handle", None):
-                capi.lib().mx_qmix_destroy(self.handle)
+                self._lib.mx_qmix_destroy(self.handle)
                 self.handle = None
         except Exception:
             pass
@@ -320,7 +321,7 @@ class QMix(object):
 
     def drop_step_graphs(self):
         for g in self._graphs.values():
-            capi.lib().mx_graph_destroy(g)
+            self._lib.mx_graph_destroy(g)
         self._graphs = {}
 
     # -- checkpoint / resume (SURVEY.md 8(f).3) ------------------------------------------------------------------------

@@ -78,6 +78,7 @@ class _Engine(object):
         h = C.c_void_p()
         capi.check(lib.mx_maddpg_create(C.byref(self.cfg), av, cv, capi.ptr(self.workspace), nbytes, C.byref(h)))
         self.handle = h
+        self._lib = lib         # the library that made the handle frees it, whichever build is bound later
         ip = lib.mx_maddpg_info(self.handle) - self.workspace.data_ptr()
         self.info = self.workspace[ip:ip + 32].view(torch.float32)
         pp = lib.mx_maddpg_priorities(self.handle) - self.workspace.data_ptr()
@@ -88,7 +89,7 @@ class _Engine(object):
 
     def close(self):
         if self.handle:
-            capi.lib().mx_maddpg_destroy(self.handle)
+            self._lib.mx_maddpg_destroy(self.handle)
             self.handle = None
 
 

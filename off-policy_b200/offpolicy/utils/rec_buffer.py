@@ -159,6 +159,7 @@ class RecPolicyBuffer(object):
         h = C.c_void_p()
         capi.check(lib.mx_replay_create(C.byref(cfg), capi.ptr(self.blob), capi.stream_ptr(), C.byref(h)))
         self.handle = h
+        self._lib = lib         # the library that made the handle frees it, even if another build is bound by the time this is collected
         self._stage = [None, None]
         self._stage_evt = [None, None]
         self._stage_i = 0
@@ -172,7 +173,7 @@ class RecPolicyBuffer(object):
     def __del__(self):
         try:
             if getattr(self, "handle", None):
-                capi.lib().mx_replay_destroy(self.handle)
+                self._lib.mx_replay_destroy(self.handle)
                 self.handle = None
         except Exception:
             pass

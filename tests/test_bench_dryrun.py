@@ -7,6 +7,7 @@ import sys
 import time
 import types
 
+import numpy as np
 import pytest
 import torch
 
@@ -60,12 +61,19 @@ CONTRACT = ["metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step
             "e2e", "gpu_launches", "roofline", "cpu_baseline", "clocks"]
 
 
-def test_mlp_workload_dry_run(bench_mod, monkeypatch):
+def _dumped(d):
+    return {p.stem: np.load(p) for p in d.glob("*.npy")}
+
+
+def test_mlp_workload_dry_run(bench_mod, monkeypatch, tmp_path):
     bench = bench_mod
     monkeypatch.setitem(bench.MLP_WORKLOADS, "mqmix_mpe_spread", (3, 18, 5, 54, 24, 600))
     monkeypatch.setattr(bench, "mlp_best_threads", lambda *a: 1)
-    args = types.SimpleNamespace(workload="mqmix_mpe_spread", impl="b200", gpus=1, steps=3, warmup=3, buffer=5000, quick=False, opt=[])
+    args = types.SimpleNamespace(workload="mqmix_mpe_spread", impl="b200", gpus=1, steps=3, warmup=3, buffer=5000, quick=False, opt=[],
+                                 dump_outputs=str(tmp_path))
     bench.run_mlp(args)
+    out = _dumped(tmp_path)
+    assert set(out) == {"loss", "grad_norm", "Q_tot", "sample_indices", "params", "target_params"} and out["sample_indices"].shape == (24,)
     line = bench._lines[-1]
     for k in CONTRACT:
         assert k in line, k
@@ -87,7 +95,12 @@ def test_recurrent_workload_dry_run(bench_mod, monkeypatch, emu_engine, workload
     monkeypatch.setitem(bench.WORKLOADS, workload, shape)
     monkeypatch.setattr(bench, "best_cpu_threads", lambda *a, **k: 1)
     monkeypatch.setattr(torch.Tensor, "pin_memory", lambda self, *a, **k: self)
-    args = types.SimpleNamespace(workload=workload, impl="b200", gpus=1, steps=3, warmup=3, buffer=48, quick=False, opt=["%s=%d" % kv for kv in opts.items()])
+
+    def eager_gpu_baseline_fails(*a, **k):          # as it does without a CUDA device; on a GPU host it would run with the stubs above
+        raise RuntimeError("no CUDA device")
+    monkeypatch.setattr(bench, "torch_eager_gpu_steps_per_s", eager_gpu_baseline_fails)
+    args = types.SimpleNamespace(workload=workload, impl="b200", gpus=1, steps=3, warmup=3, buffer=48, quick=False, opt=["%s=%d" % kv for kv in opts.items()],
+                                 dump_outputs=None)
     for k, v in opts.items():
         emu_engine.lib().mx_set_option(k.encode(), v)
     try:
@@ -103,18 +116,37 @@ def test_recurrent_workload_dry_run(bench_mod, monkeypatch, emu_engine, workload
     assert line["config"]["workload"] == workload
     assert line["gpu_launches"] > 0 and line["e2e"]["h2d_bytes_per_step"] > 0 and line["e2e"]["lagged_read_value"] > 0
     assert line["roofline"]["kernel"] in line["kernels"]
-    assert line["torch_eager_gpu_baseline"]["value"] is None          # no CUDA device here: the secondary baseline is skipped, the line survives
+    assert line["torch_eager_gpu_baseline"]["value"] is None          # the secondary baseline failed: it is skipped, the line survives
+
+
+def test_dump_outputs_repeat_and_follow_the_step_count(bench_mod, monkeypatch, emu_engine, tmp_path):
+    """--dump-outputs on the default arm: float32 / float64 arrays of the last timed step, identical in two runs with the same arguments,
+    different after one more timed step."""
+    bench = bench_mod
+    monkeypatch.setitem(bench.WORKLOADS, "qmix_mpe_spread", (3, 18, 5, 54, 5, 4, False))
+    runs = []
+    for k, steps in enumerate((3, 3, 4)):
+        args = types.SimpleNamespace(workload="qmix_mpe_spread", impl="b200", gpus=1, steps=steps, warmup=3, buffer=48, quick=True, opt=[],
+                                     dump_outputs=str(tmp_path / str(k)))
+        bench.run_engine(args)
+        runs.append(_dumped(tmp_path / str(k)))
+    assert set(runs[0]) == {"loss", "grad_norm", "Q_tot", "sample_indices", "params", "target_params"}
+    for name, a in runs[0].items():
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, runs[1][name]), name
+    assert not np.array_equal(runs[0]["params"], runs[2]["params"])
 
 
 @pytest.mark.parametrize("workload,shape", [("rmatd3_spread", (2, 6, 2, 8, 4, 4, True, False)), ("rmaddpg_spread_disc", (2, 6, 3, 8, 4, 4, False, True))])
-def test_maddpg_workload_dry_run(bench_mod, monkeypatch, emu_engine, workload, shape):
+def test_maddpg_workload_dry_run(bench_mod, monkeypatch, emu_engine, workload, shape, tmp_path):
     """The R-MADDPG / R-MATD3 bench arm (run_maddpg) at shrunken shapes: Box + TD3 target noise, Discrete + Gumbel noise.  The engine side
     takes its configuration from the package (factory.MaddpgLearnerConfig); the oracle is imported for the CPU baseline only."""
     bench = bench_mod
     monkeypatch.setitem(bench.MADDPG_WORKLOADS, workload, shape)
     monkeypatch.setattr(torch.Tensor, "pin_memory", lambda self, *a, **k: self)
-    args = types.SimpleNamespace(workload=workload, impl="b200", gpus=1, steps=3, warmup=3, buffer=48, quick=False, opt=[])
+    args = types.SimpleNamespace(workload=workload, impl="b200", gpus=1, steps=3, warmup=3, buffer=48, quick=False, opt=[], dump_outputs=str(tmp_path))
     bench.run_maddpg(args)
+    out = _dumped(tmp_path)
+    assert {"critic_loss", "critic_grad_norm", "sample_indices", "actor_params", "target_actor_params", "critic_params", "target_critic_params"} <= set(out)
     line = bench._lines[-1]
     for k in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "config", "e2e", "gpu_launches", "cpu_baseline"):
         assert k in line, k

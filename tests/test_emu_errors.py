@@ -109,6 +109,35 @@ def test_trainer_rejects_what_it_does_not_implement(emu_engine):
         RecReplayBuffer({"policy_0": info}, {"policy_0": [0, 1, 2]}, 8, 4, False, True)               # use_same_share_obs=False
 
 
+def test_objects_are_freed_by_the_library_that_made_them(emu_engine, monkeypatch):
+    """A replay, learner or step graph collected after another build of the library was bound (a process that uses the emulated build
+    and then the CUDA one) hands its handle back to the build that made it: the other build would be given a pointer it never issued."""
+    import gc
+    from offpolicy._b200 import factory
+    from offpolicy._b200.graph import StepGraph
+    N, O, A, S, T = 2, 4, 3, 5, 3
+    buf = factory.make_rec_buffers(N, O, A, S, T, 8, rng="device", max_batch=4)
+    buf.insert(4, *_episodes(N, O, A, S, T, 4, np.random.RandomState(2)))
+    args, pol, tr = qc.build_trainer(QmixConfig(n_agents=N, obs_dim=O, act_dim=A, state_dim=S), 4, T)
+    graph = StepGraph(buf, tr, 4)
+    margs, mpol, mtr = factory.build_maddpg(factory.MaddpgLearnerConfig(n_agents=2, obs_dim=5, act_dim=2, state_dim=6), 4, T)
+    lib, freed = emu_engine.lib(), []
+    names = ("mx_graph_destroy", "mx_qmix_destroy", "mx_replay_destroy", "mx_maddpg_destroy")
+    for name in names:
+        monkeypatch.setattr(lib, name, lambda h, _f=getattr(lib, name), _n=name: (freed.append(_n), _f(h))[1])
+
+    class OtherBuild(object):
+        calls = []
+
+        def __getattr__(self, name):
+            self.calls.append(name)
+            return lambda *a: 0
+    monkeypatch.setattr(emu_engine, "_lib", OtherBuild())
+    del buf, args, pol, tr, graph, margs, mpol, mtr
+    gc.collect()
+    assert OtherBuild.calls == [] and set(freed) == set(names), (OtherBuild.calls, freed)
+
+
 def test_c_abi_status_codes(emu_engine):
     lib = emu_engine.lib()
     cfg = emu_engine.ReplayCfg(0, 4, 2, 3, 3, 2, 1, 0, 0, 4, 0.0)          # capacity 0
